@@ -18,8 +18,15 @@ buffered against the compute of the neighbouring steps.  `roofline` is for the
 dominant kernel (the heads' 3x3 implicit-GEMM launch), timed live with CUDA
 events on the launching stream (cp_plan_profile); `cpu_baseline` is the CPU
 oracle (a port of the reference algorithm, see oracle/) on a bounded sample.
+
+The heat-map biases of the seeded weights are calibrated, before anything is
+timed, on the reference graph in PyTorch (deterministic fp32, torchvision's
+deform_conv2d for the DCNv2 layers), so every build sees the same weights and
+inputs; bench.py therefore needs torchvision.  `--dump-outputs DIR` writes what
+the last timed step returned, so two builds can be compared output for output.
 """
 import argparse
+import contextlib
 import json
 import os
 import subprocess
@@ -48,6 +55,7 @@ GFLOP_PER_IMAGE = 85.11          # BASELINE.md section 2 (reference graph, 2*MAC
 HEAD_GAIN = 1.0
 TARGET_OBJECTS = 4               # centre peaks per frame that pass vis_thresh after bias calibration (Objectron-like density)
 N_ROTATE = 6                     # distinct input batches rotated through (6 x 25 MB uint8 + activations >> 126 MB L2)
+DUMP_LIMIT = 64 << 20            # bytes written by --dump-outputs
 
 
 def load_peaks():
@@ -117,11 +125,56 @@ class ClockSampler(threading.Thread):
                 "reasons": reasons, "samples": len(self.samples)}
 
 
-def calibrate_head_bias(model, eng, x, target=TARGET_OBJECTS):
-    """Setup only, outside any timed region: see centerpose_b200.synth.calibrate_head_bias."""
+@contextlib.contextmanager
+def torch_graph_on_gpu(allow_tf32, deterministic=False):
+    """The reference graph (oracle/net_ref.py: torch / cuDNN convolutions, BatchNorm, torchvision.ops.deform_conv2d for
+    the DCNv2 layers -- the `_ext` stand-in of SURVEY.md Appendix E) on the GPU.  Yields the net_ref module."""
+    from oracle import net_ref
+    try:
+        import torchvision
+    except ImportError as e:
+        raise RuntimeError("bench.py needs torchvision: its deform_conv2d runs the DCNv2 layers of the PyTorch reference "
+                           "graph, which calibrates the benchmark's heat-map biases") from e
+    cudnn = torch.backends.cudnn
+    orig = net_ref.dcn_v2_forward_ref
+    net_ref.dcn_v2_forward_ref = lambda a, off, mask, w, b: torchvision.ops.deform_conv2d(a, off, w, b, padding=1, mask=mask)
+    old = (cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32, cudnn.benchmark, cudnn.deterministic)
+    cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = bool(allow_tf32)
+    cudnn.benchmark, cudnn.deterministic = not deterministic, deterministic
+    try:
+        yield net_ref
+    finally:
+        net_ref.dcn_v2_forward_ref = orig
+        cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32, cudnn.benchmark, cudnn.deterministic = old
+
+
+def calibrate_head_bias(model, sd, opt, x, target=TARGET_OBJECTS):
+    """Setup only, outside any timed region: see centerpose_b200.synth.calibrate_head_bias.  The heads it reads come
+    from the reference graph in PyTorch (fp32, deterministic cuDNN algorithms), not from this project's kernels, so the
+    calibrated weights -- and with them every input of the timed steps -- are the same whichever build runs."""
     from centerpose_b200 import synth
-    synth.calibrate_head_bias(model, eng.forward(x), target)
+    sdg = {k: v.to(x.device) for k, v in sd.items()}
+    with torch_graph_on_gpu(allow_tf32=False, deterministic=True) as net_ref:
+        heads = net_ref.forward(x, sdg, opt.heads, "dla_34")
+    synth.calibrate_head_bias(model, heads, target)
     return model
+
+
+def dump_outputs(out_dir, poses, n_valid):
+    """Writes the pose records [frames, K, 192] and detection counts [frames] of one step as float32 .npy files.  The
+    kernels leave the records past a frame's n_valid unwritten (they hold an earlier step's values), so those are
+    zeroed: two builds compare on defined values only.  Above DUMP_LIMIT a fixed, seeded sample of frames is written;
+    frame_index.npy names the frames kept."""
+    poses = poses.cpu().numpy().copy()
+    n_valid = n_valid.cpu().numpy()
+    poses[np.arange(poses.shape[1])[None, :] >= n_valid[:, None]] = 0.0
+    n = poses.shape[0]
+    keep = min(n, (DUMP_LIMIT - 4096) // (poses[0].nbytes + 4 + 8))
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "poses.npy"), poses[idx])
+    np.save(os.path.join(out_dir, "n_valid.npy"), n_valid[idx].astype(np.float32))
+    np.save(os.path.join(out_dir, "frame_index.npy"), idx.astype(np.float64))
 
 
 def cpu_reference_step(sd, opt, frames_u8, cam, budget_s=None, stages=None):
@@ -162,32 +215,20 @@ def cpu_reference_step(sd, opt, frames_u8, cam, budget_s=None, stages=None):
 
 
 def gpu_torch_forward_ms(sd, opt, x, allow_tf32, reps=10):
-    """BASELINE config 2 baseline leg: the reference graph (oracle/net_ref.py: torch / cuDNN convolutions, BatchNorm,
-    torchvision.ops.deform_conv2d for the DCNv2 layers -- the `_ext` stand-in of SURVEY.md Appendix E) on the GPU.
+    """BASELINE config 2 baseline leg: the reference graph on the GPU (torch_graph_on_gpu).
     Returns (ms per forward, heads)."""
-    from oracle import net_ref
-    import torchvision
     sdg = {k: v.to(x.device) for k, v in sd.items()}
-    orig = net_ref.dcn_v2_forward_ref
-    net_ref.dcn_v2_forward_ref = lambda a, off, mask, w, b: torchvision.ops.deform_conv2d(a, off, w, b, padding=1, mask=mask)
-    old = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.benchmark)
-    torch.backends.cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = bool(allow_tf32)
-    torch.backends.cudnn.benchmark = True
-    try:
-        with torch.no_grad():
-            for _ in range(3):
-                out = net_ref.forward(x, sdg, opt.heads, "dla_34")
-            torch.cuda.synchronize()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            for _ in range(reps):
-                out = net_ref.forward(x, sdg, opt.heads, "dla_34")
-            e1.record()
-            torch.cuda.synchronize()
-        return e0.elapsed_time(e1) / reps, out
-    finally:
-        net_ref.dcn_v2_forward_ref = orig
-        torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.benchmark = old
+    with torch_graph_on_gpu(allow_tf32) as net_ref, torch.no_grad():
+        for _ in range(3):
+            out = net_ref.forward(x, sdg, opt.heads, "dla_34")
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(reps):
+            out = net_ref.forward(x, sdg, opt.heads, "dla_34")
+        e1.record()
+        torch.cuda.synchronize()
+    return e0.elapsed_time(e1) / reps, out
 
 
 def extra_configs(args, det, eng32, sd, opt, cam, dev, ev_time):
@@ -331,7 +372,11 @@ def main():
     ap.add_argument("--no-fast-mode", action="store_true", help="skip the extra single-pass tf32 measurement")
     ap.add_argument("--no-extra-configs", action="store_true",
                     help="skip the BASELINE.json configs 1 / 2 / 5 legs (batch-1 latency vs PyTorch-GPU, dlav1_34, tracking)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step returned (pose records, detection counts) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     if args.warmup < 3:
@@ -364,10 +409,9 @@ def main():
     model.load_state_dict(sd)
     det = cpb.ObjectPoseDetector(opt, model=model)
     cam = synth.default_camera(512, 512)
-    eng = det.model.engine(B, 512, 512, dev)
     calib = torch.from_numpy(synth.normalize_frames(synth.synthetic_frames(B, 512, 512, seed=317 + 1000 * rank))).to(dev)
-    calibrate_head_bias(det.model, eng, calib)
-    eng = det.model.engine(B, 512, 512, dev)            # re-ingests the calibrated weights
+    calibrate_head_bias(det.model, sd, opt, calib)
+    eng = det.model.engine(B, 512, 512, dev)            # with the calibrated weights
     sd = {k: v.detach().cpu() for k, v in det.model.state_dict().items()}
     del calib
     prm = decode_params(opt)
@@ -432,6 +476,8 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     ms_res = timed(step_resident, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *pbuf.views(pbuf.gathered))
     clocks = sampler
     ms_e2e = timed(step_e2e, args.steps, args.warmup, drain=drain_e2e)
     sampler.stop_flag = True

@@ -14,6 +14,13 @@ Fixtures
                 pnp_shell results of the reference on planted head tensors
                 (torch==1.1.0 comparison semantics, see ref_shims.legacy_bool_arith)
   dcn_*.npz     the reference's own C++ CPU deformable-conv (oracle/_ref) outputs
+  reference_opts.json, state_dict_keys.json
+                the options `opts().parse / init` derives the way src/demo.py sets them up, and the
+                state-dict keys / shapes of `create_model`, per model configuration
+  gpfit_moments.npz
+                `utils/gpfit.py` moments() and fitgaussian() on seeded 11 x 11 windows
+  demo_frame_0.json
+                the --debug 4 JSON the unmodified src/demo.py writes for tests/data/frame_0.png
 """
 import copy
 import os
@@ -31,6 +38,10 @@ from centerpose_b200 import synth     # noqa: E402
 from centerpose_b200 import _lib as L  # noqa: E402  (record layout constants only)
 
 GOLD = os.path.join(ROOT, "tests", "golden")
+# CPU threads of every reference run here.  oneDNN's fp32 convolutions sum in an order that depends on the thread count,
+# and the random-weight graphs amplify that to ~1e-4 of max|head|, so the tests run the oracle with the same count
+# (tests/util.py golden_threads) and hold it to the fixtures at the level of fp32 round-off.
+GOLDEN_THREADS = 8
 
 NET_CASES = [
     # name, arch, tracking, batch, H, W, weight seed, input seed
@@ -60,6 +71,10 @@ DECODE_CASES = [
     ("decode_scale075_rep1_3obj", False, 1, 3, 0.5, 2, 81, "chair", (), False, {"test_scales": [0.75, 1.0]}),
     # a single scale != 1 with --nms off: division only; rep_mode 0 feeds the divided `kps` to the PnP
     ("decode_scale125_rep0_nonms", False, 0, 4, 1.0, 1, 91, "cup", (), False, {"test_scales": [1.25], "nms": False}),
+    # one frame each: five objects 2 px apart in their two keypoint estimates, the tracking heads, rep_mode 3
+    ("decode_rep1_5obj", False, 1, 5, 2.0, 1, 77, "chair"),
+    ("decode_track_rep1_2obj", True, 1, 2, 0.5, 1, 78, "chair"),
+    ("decode_rep3_3obj", False, 3, 3, 1.0, 1, 79, "chair"),
 ]
 
 
@@ -284,12 +299,102 @@ def make_dcn_bwd():
         print(name, {k: float(np.abs(v).max()) for k, v in out.items()})
 
 
+# (arch, tracking task, rep_mode); state-dict keys are recorded for rep_mode 1
+MODEL_CASES = [("dla_34", False, 1), ("dlav1_34", False, 1), ("dla_34", True, 1), ("dlav1_34", False, 0)]
+OPT_FIELDS = ("K", "rep_mode", "vis_thresh", "nms", "use_pnp", "head_conv", "down_ratio", "mean", "std", "c", "input_h",
+              "input_w", "num_classes", "test_scales", "fix_res", "hm_hp", "reg_offset", "reg_hp_offset", "tracking_task",
+              "hps_uncertainty", "obj_scale_uncertainty", "balance_coefficient")
+
+
+def model_key(arch, tracking):
+    return "%s_%s" % (arch, "track" if tracking else "plain")
+
+
+def make_reference_models():
+    import json
+    from lib.models.model import create_model as ref_create
+    opts, keys = {}, {}
+    for arch, trk, rep in MODEL_CASES:
+        r = ref_shims.make_opt(arch, tracking_task=trk, rep_mode=rep)
+        opts["%s_rep%d" % (model_key(arch, trk), rep)] = dict(heads=[[k, v] for k, v in r.heads.items()],
+                                                              **{f: getattr(r, f) for f in OPT_FIELDS})
+        if rep == 1:
+            m = ref_create(r.arch, r.heads, r.head_conv, r)
+            keys[model_key(arch, trk)] = [[k, list(v.shape)] for k, v in m.state_dict().items()]
+    for name, d in (("reference_opts.json", opts), ("state_dict_keys.json", keys)):
+        with open(os.path.join(GOLD, name), "w") as f:
+            json.dump(d, f)
+        print(name, list(d))
+
+
+def gpfit_windows():
+    """30 seeded 11 x 11 heat-map windows: a Gaussian bump off the pixel grid times uniform noise."""
+    rng = np.random.default_rng(3)
+    g = np.exp(-((np.arange(11)[:, None] - 5.3) ** 2 + (np.arange(11)[None] - 4.6) ** 2) / 6)
+    return [rng.random((11, 11)) * g for _ in range(30)]
+
+
+def make_gpfit():
+    from lib.utils.gpfit import moments, fitgaussian
+    ws = gpfit_windows()
+    np.savez_compressed(os.path.join(GOLD, "gpfit_moments.npz"), moments=np.array([moments(w) for w in ws]),
+                        fitgaussian=np.array([fitgaussian(w) for w in ws]))
+    print("gpfit_moments", len(ws))
+
+
+DEMO_FRAME = os.path.join(ROOT, "tests", "data", "frame_0.png")
+# src/demo.py's camera matrix when --cam_intrinsic is not given
+DEMO_CAMERA = np.array([[663.0287679036459, 0, 300.2775065104167], [0, 663.0287679036459, 395.00066121419275], [0, 0, 1]])
+
+
+def demo_checkpoint(path):
+    """Seeded dla_34 weights whose heat-map biases let a few centres pass vis_thresh on DEMO_FRAME, saved the way the
+    reference saves checkpoints."""
+    import cv2
+    import centerpose_b200 as cpb
+    from oracle import net_ref
+    from oracle import preprocess_ref as pr
+    opt = cpb.default_opt("dla_34")
+    m = cpb.create_model(opt.arch, opt.heads, opt.head_conv, opt)
+    m.load_state_dict(synth.seeded_state_dict(m, seed=9, offset_std=0.3, head_gain=6.0))
+    # the reference pre-process at 512 x 512 (cv2), then calibrate the two heat-map biases on the oracle heads
+    x = torch.from_numpy(pr.pre_process(cv2.imread(DEMO_FRAME), 512, 512, opt.mean, opt.std))
+    sd = {k: v.detach() for k, v in m.state_dict().items()}
+    synth.calibrate_head_bias(m, net_ref.forward(x, sd, opt.heads, "dla_34"), target=10)
+    cpb.save_model(path, 1, m)
+    return path
+
+
+def make_demo():
+    """The unmodified src/demo.py on the CPU (torch-1.1 comparison semantics, see DESIGN.md section 5)."""
+    import json
+    import runpy
+    import tempfile
+    with tempfile.TemporaryDirectory() as tmp:
+        out = os.path.join(tmp, "ref") + "/"
+        argv = ["--demo", DEMO_FRAME, "--arch", "dla_34", "--load_model", demo_checkpoint(os.path.join(tmp, "ck.pth")),
+                "--debug", "4", "--c", "shoe", "--gpus", "-1", "--demo_save", out]
+        saved_argv, saved_cwd = sys.argv, os.getcwd()
+        sys.argv = ["demo.py"] + argv
+        os.chdir(ref_shims.REF_SRC)
+        try:
+            with ref_shims.legacy_bool_arith():
+                runpy.run_path(os.path.join(ref_shims.REF_SRC, "demo.py"), run_name="__main__")
+        finally:
+            sys.argv = saved_argv
+            os.chdir(saved_cwd)
+        j = json.load(open(os.path.join(out, "frame_0", "frame_0.json")))
+    with open(os.path.join(GOLD, "demo_frame_0.json"), "w") as f:
+        json.dump(j, f)
+    print("demo_frame_0", len(j["objects"]), "objects")
+
+
 if __name__ == "__main__":
     if not ref_shims.reference_available():
         raise SystemExit("reference tree not present: goldens can only be generated in the build container")
     ref_shims.install()
     os.makedirs(GOLD, exist_ok=True)
-    torch.set_num_threads(os.cpu_count() or 1)
+    torch.set_num_threads(GOLDEN_THREADS)
     only = set(sys.argv[1:])
     if not only:
         make_dcn()
@@ -298,3 +403,9 @@ if __name__ == "__main__":
     make_net(only)
     if not only or any(n.startswith("decode_") for n in only):
         make_decode(only)
+    if not only or "models" in only:
+        make_reference_models()
+    if not only or "gpfit" in only:
+        make_gpfit()
+    if not only or "demo" in only:
+        make_demo()

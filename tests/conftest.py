@@ -48,13 +48,3 @@ def pose_host():
         os.makedirs(out_dir, exist_ok=True)
         subprocess.check_call(["g++", "-O2", "-shared", "-fPIC", "-o", so, src])
     return ctypes.CDLL(so)
-
-
-@pytest.fixture(scope="session")
-def reference():
-    """The unmodified reference through oracle/ref_shims (build container only)."""
-    from oracle import ref_shims
-    if not ref_shims.reference_available():
-        pytest.skip("/root/reference is not present on this box")
-    ref_shims.install()
-    return ref_shims

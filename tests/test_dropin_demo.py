@@ -1,21 +1,15 @@
-"""Drop-in proof (VERDICT r01 item 10, SURVEY.md rows a-12 / b / f-3): the reference's own `src/demo.py`, UNMODIFIED, is
-run twice through `runpy` on the same image and checkpoint --
-
-  arm A: the unmodified reference (`lib.*` as shipped, CPU, `--gpus -1`),
-  arm B: after `centerpose_b200.dropin.install()`: `lib.models.model` / `lib.detectors.detector_factory` resolve to this
-         package, so demo.py builds OUR ObjectPoseDetector from the reference's own `opts().parse / init` Namespace and
-         calls OUR `run()` (pre_process, result structures, dict_out, save_results).
-
-and the JSON files both arms write with `--debug 4` (object_pose.py:357-414) are compared key by key.  There is no GPU
-in the build container, so in arm B the two device stages (`DLASegB200.forward`, `cp_decode_pnp`) are replaced by the CPU
-oracle (test infrastructure) -- everything else of arm B is the product's host code.  On the GPU box (no reference tree
-there) `test_demo_flow_on_gpu` runs the same flow with the real engine on the committed sample frames.
+"""Drop-in proof (SURVEY.md rows a-12 / b / f-3): the flow of the reference's `src/demo.py` (demo.py:22-87:
+`detector_factory[opt.task](opt)` from a checkpoint path, then `run(image path, meta_inp)` with `--debug 4`) on this
+package's ObjectPoseDetector -- pre_process, result structures, dict_out, save_results -- must write the JSON file the
+unmodified reference wrote for the same frame, checkpoint and arguments (tests/golden/demo_frame_0.json, recorded by
+oracle/make_golden.py from the reference's own demo.py on the CPU).  The JSON is compared key by key.  Without a GPU the
+two device stages (`DLASegB200.forward`, `cp_decode_pnp`) are replaced by the CPU oracle (test infrastructure) --
+everything else is the product's host code.  `test_demo_flow_on_gpu` runs the same flow with the real engine on the
+committed sample frames.
 """
 import copy
 import json
 import os
-import runpy
-import sys
 
 import numpy as np
 import pytest
@@ -27,6 +21,7 @@ from centerpose_b200 import synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 FRAME = os.path.join(ROOT, "tests", "data", "frame_0.png")
+GOLD = os.path.join(ROOT, "tests", "golden")
 OBJECT_KEYS = {"class", "ct", "bbox", "confidence", "kps_displacement_mean", "kps_heatmap_mean", "kps_heatmap_std",
                "kps_heatmap_height", "obj_scale", "location", "quaternion_xyzw", "kps_pnp", "kps_3d_cam"}
 
@@ -62,59 +57,39 @@ def _oracle_process(self, images, pre_images=None, pre_hms=None, pre_hm_hp=None,
 
 @pytest.fixture(scope="module")
 def checkpoint(tmp_path_factory):
-    """Seeded dla_34 weights whose heat-map biases let a few centres pass vis_thresh on the sample frame, saved the way
-    the reference saves checkpoints."""
-    from oracle import net_ref
-    import cv2
-    opt = cpb.default_opt("dla_34")
-    m = cpb.create_model(opt.arch, opt.heads, opt.head_conv, opt)
-    m.load_state_dict(synth.seeded_state_dict(m, seed=9, offset_std=0.3, head_gain=6.0))
-    img = cv2.imread(FRAME)
-    # the reference pre-process at 512 x 512 (cv2), then calibrate the two heat-map biases on the oracle heads
-    from oracle import preprocess_ref as pr
-    x = torch.from_numpy(pr.pre_process(img, 512, 512, opt.mean, opt.std))
-    sd = {k: v.detach() for k, v in m.state_dict().items()}
-    synth.calibrate_head_bias(m, net_ref.forward(x, sd, opt.heads, "dla_34"), target=10)
-    path = str(tmp_path_factory.mktemp("ckpt") / "chair_seeded.pth")
-    cpb.save_model(path, 1, m)
-    return path
+    from oracle.make_golden import demo_checkpoint
+    from tests.util import golden_threads
+    with golden_threads():
+        return demo_checkpoint(str(tmp_path_factory.mktemp("ckpt") / "chair_seeded.pth"))
 
 
-def _run_demo(argv, cwd):
-    saved_argv, saved_cwd = sys.argv, os.getcwd()
-    sys.argv = ["demo.py"] + argv
-    os.chdir(cwd)
-    try:
-        runpy.run_path("/root/reference/src/demo.py", run_name="__main__")
-    finally:
-        sys.argv = saved_argv
-        os.chdir(saved_cwd)
+class _RecordingDebugger(object):
+    """Stands in for the reference's Debugger (drawing), which only exists inside the reference tree."""
+
+    def __init__(self):
+        self.calls = []
+
+    def __getattr__(self, name):
+        return lambda *a, **k: self.calls.append(name)
 
 
-def test_demo_py_runs_unchanged_on_the_dropin(reference, checkpoint, tmp_path, monkeypatch):
-    from centerpose_b200 import dropin
-    src = "/root/reference/src"
-    monkeypatch.syspath_prepend(src)
-    out_a, out_b = str(tmp_path / "ref") + "/", str(tmp_path / "ours") + "/"
-    common = ["--demo", FRAME, "--arch", "dla_34", "--load_model", checkpoint, "--debug", "4", "--c", "shoe"]
-    # ---- arm A: the unmodified reference on the CPU (torch-1.1 comparison semantics, see DESIGN.md section 5)
-    with reference.legacy_bool_arith():
-        _run_demo(common + ["--gpus", "-1", "--demo_save", out_a], src)
-    ja = json.load(open(os.path.join(out_a, "frame_0", "frame_0.json")))
-    # ---- arm B: same script, same argv, our package behind the reference's import names
-    saved = {k: sys.modules.get(k) for k in ("lib.models.model", "lib.detectors.detector_factory", "_ext")}
-    try:
-        dropin.install(ext=False)
-        monkeypatch.setattr(cpb.ObjectPoseDetector, "process", _oracle_process)
-        monkeypatch.setattr(cpb.ObjectPoseDetector, "_to_device", lambda self, t: t)
-        _run_demo(common + ["--gpus", "0", "--demo_save", out_b], src)
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
-    jb = json.load(open(os.path.join(out_b, "frame_0", "frame_0.json")))
+def test_demo_flow_matches_reference_json(checkpoint, tmp_path, monkeypatch):
+    from oracle.make_golden import DEMO_CAMERA
+    from tests.util import golden_threads
+    ja = json.load(open(os.path.join(GOLD, "demo_frame_0.json")))
+    opt = cpb.default_opt("dla_34", c="shoe", debug=4, load_model=checkpoint)
+    opt.demo = FRAME
+    opt.demo_save = str(tmp_path / "ours")
+    dbg = _RecordingDebugger()
+    monkeypatch.setattr(cpb.ObjectPoseDetector, "process", _oracle_process)
+    monkeypatch.setattr(cpb.ObjectPoseDetector, "_to_device", lambda self, t: t)
+    monkeypatch.setattr(cpb.ObjectPoseDetector, "_debugger", lambda self, debugger: dbg)
+    monkeypatch.setattr(torch.cuda, "synchronize", lambda *a, **k: None)      # run()'s timing stamps; no device here
+    det = cpb.detector_factory[opt.task](opt)
+    det.pause = False
+    with golden_threads():
+        det.run(FRAME, meta_inp={"camera_matrix": DEMO_CAMERA})
+    jb = json.load(open(os.path.join(opt.demo_save, "frame_0", "frame_0.json")))
     # ---- same schema, same objects
     assert set(ja) == set(jb) == {"camera_data", "objects"}
     assert np.allclose(ja["camera_data"], jb["camera_data"])
@@ -128,15 +103,15 @@ def test_demo_py_runs_unchanged_on_the_dropin(reference, checkpoint, tmp_path, m
             if k == "quaternion_xyzw" and np.dot(a, b) < 0:
                 b = -b
             # The keypoints of a random-weight network are not a projected cuboid, so the PnP problem is far from
-            # consistent and cv2's LM (arm A) and the restated LM (arm B, 20-iteration cap, DESIGN.md section 4) stop at
-            # slightly different points: the four PnP outputs get a loose bound here; on consistent keypoints the two
-            # agree to 1e-6 (tests/test_pose_core_host.py, tests/test_oracle_decode.py).
+            # consistent and cv2's LM (the reference) and the restated LM (20-iteration cap, DESIGN.md section 4) stop
+            # at slightly different points: the four PnP outputs get a loose bound here; on consistent keypoints the
+            # two agree to 1e-6 (tests/test_pose_core_host.py, tests/test_oracle_decode.py).
             tol = {"quaternion_xyzw": 5e-2, "location": 5e-2, "kps_3d_cam": 5e-2, "kps_pnp": 5e-2, "confidence": 1e-5,
                    "kps_heatmap_height": 1e-5, "obj_scale": 1e-5}.get(k, 2e-3)      # pixels: fp32 records
             scale = max(1.0, np.abs(a).max()) if k in ("location", "kps_3d_cam", "kps_pnp") else 1.0
             assert np.abs(a - b).max() <= tol * scale, (k, float(np.abs(a - b).max()))
-    # the rendered image exists in both arms (the reference's Debugger is importable inside its tree)
-    assert any(f.endswith(".png") for f in os.listdir(os.path.join(out_b, "frame_0")))
+    # the frame is drawn and saved next to the JSON, as the reference does
+    assert "save_all_imgs_demo" in dbg.calls
 
 
 @pytest.mark.gpu

@@ -44,15 +44,9 @@ def _golden_512():
 @functools.lru_cache(maxsize=None)
 def _truth_512():
     """fp64 CPU evaluation of the oracle graph on the golden's input (once per session, ~1 min)."""
-    import os
     from oracle import net_ref
-    from tests.util import GOLD
     g, x = _golden_512()
     opt = cpb.default_opt("dla_34")
-    cache = os.path.join(GOLD, "_cache", "net_dla34_b1_512_truth64.npz")     # git-ignored, written in the build container
-    if os.path.exists(cache):
-        z = np.load(cache)
-        return {h: z[h] for h in opt.heads}
     m = cpb.create_model(opt.arch, opt.heads, opt.head_conv, opt)
     sd = synth.seeded_state_dict(m, seed=int(g["wseed"]), offset_std=float(g["offset_std"]))
     sd64 = {k: (v.double() if v.dtype.is_floating_point else v) for k, v in sd.items()}

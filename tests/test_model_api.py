@@ -22,16 +22,16 @@ def test_state_dict_matches_reference(arch, trk, key, n):
     assert got == want          # same keys, same shapes, same order
 
 
-def test_state_dict_matches_live_reference(reference):
-    from lib.models.model import create_model as ref_create
+def test_state_dict_matches_live_reference():
+    """Same heads (names, channels, order) as the reference's options and the same state dict as its create_model."""
+    ref = json.load(open(os.path.join(GOLD, "reference_opts.json")))
+    keys = json.load(open(os.path.join(GOLD, "state_dict_keys.json")))
     for arch, trk in (("dla_34", False), ("dlav1_34", False), ("dla_34", True)):
-        ropt = reference.make_opt(arch, tracking_task=trk)
-        r = ref_create(ropt.arch, ropt.heads, ropt.head_conv, ropt)
+        key = "%s_%s" % (arch, "track" if trk else "plain")
         opt = cpb.default_opt(arch, tracking_task=trk)
-        assert list(opt.heads.items()) == list(ropt.heads.items())
+        assert [[k, v] for k, v in opt.heads.items()] == ref[key + "_rep1"]["heads"]
         m = cpb.create_model(opt.arch, opt.heads, opt.head_conv, opt)
-        assert [(k, tuple(v.shape)) for k, v in m.state_dict().items()] == \
-               [(k, tuple(v.shape)) for k, v in r.state_dict().items()]
+        assert [[k, list(v.shape)] for k, v in m.state_dict().items()] == keys[key]
 
 
 def test_save_load_roundtrip(tmp_path, capsys):
@@ -90,15 +90,17 @@ def test_dropin_registers_reference_module_names():
                 sys.modules[k] = v
 
 
-def test_default_opt_matches_reference(reference):
+def test_default_opt_matches_reference():
+    """default_opt() vs the options the reference derives the way src/demo.py sets them up (oracle/make_golden.py)."""
+    ref = json.load(open(os.path.join(GOLD, "reference_opts.json")))
     for arch, trk, rep in (("dla_34", False, 1), ("dla_34", True, 1), ("dlav1_34", False, 0)):
-        r = reference.make_opt(arch, tracking_task=trk, rep_mode=rep)
+        r = ref["%s_%s_rep%d" % (arch, "track" if trk else "plain", rep)]
         o = cpb.default_opt(arch, tracking_task=trk, rep_mode=rep)
         for f in ("K", "rep_mode", "vis_thresh", "nms", "use_pnp", "head_conv", "down_ratio", "mean", "std", "c",
                   "input_h", "input_w", "num_classes", "test_scales", "fix_res", "hm_hp", "reg_offset",
                   "reg_hp_offset", "tracking_task", "hps_uncertainty", "obj_scale_uncertainty"):
-            assert getattr(o, f) == getattr(r, f), f
-        assert o.balance_coefficient == r.balance_coefficient
+            assert getattr(o, f) == r[f], f
+        assert o.balance_coefficient == r["balance_coefficient"]
 
 
 def test_seeded_weights_are_deterministic():

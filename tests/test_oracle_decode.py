@@ -1,6 +1,6 @@
 """Pins oracle/decode_ref.py + oracle/pnp_ref.py against the golden vectors the
-unmodified reference produced (tests/golden/decode_*.npz), against the live
-reference when present, and against cv2.solvePnPGeneric directly."""
+unmodified reference produced (tests/golden/decode_*.npz, gpfit_moments.npz) and
+against cv2.solvePnPGeneric directly."""
 import copy
 
 import numpy as np
@@ -24,8 +24,7 @@ def _params(g):
                                    nms=nms, num_scales=len(scales))
 
 
-@pytest.mark.parametrize("name", CASES)
-def test_oracle_matches_reference_golden(name):
+def _check_golden(name):
     g = golden(name)
     hb, truths = decode_case_inputs(g)
     prm = _params(g)
@@ -43,20 +42,16 @@ def test_oracle_matches_reference_golden(name):
         compare_records(recs, want_recs, L, tol_px=1e-9, tol_q=1e-6)
 
 
-def test_oracle_matches_live_reference(reference):
-    from oracle.make_golden import reference_pipeline
-    for trk, rep, nobj, dis, seed in ((False, 1, 5, 2.0, 77), (True, 1, 2, 0.5, 78), (False, 3, 3, 1.0, 79)):
-        opt = reference.make_opt("dla_34", tracking_task=trk, rep_mode=rep)
-        heads = synth.TRACKING_HEADS if trk else synth.DEFAULT_HEADS
-        h, truth = synth.planted_heads(n_obj=nobj, seed=seed, heads=heads, disagree_px=dis)
-        c, s = np.array([256., 256.], np.float32), 512.0
-        ref_dets, ref_recs = reference_pipeline(h, opt, truth["cam"], 512, 512, c, s)
-        prm = decode_ref.DecodeParams(rep_mode=rep, use_moments=trk, vis_thresh=opt.vis_thresh, category=opt.c)
-        dets, recs = oracle_records(h, prm, truth["cam"], 512, 512, c, s, L)
-        valid = ref_dets["scores"][0, :, 0] > 0.05
-        for k in DETS_KEYS:
-            assert np.abs(dets[k][valid] - ref_dets[k][0][valid]).max() <= 2e-6, k
-        compare_records(recs, ref_recs, L, tol_px=1e-9, tol_q=1e-6)
+@pytest.mark.parametrize("name", CASES)
+def test_oracle_matches_reference_golden(name):
+    _check_golden(name)
+
+
+def test_oracle_matches_live_reference():
+    """Three single planted frames -- five objects whose two keypoint estimates disagree by 2 px, the tracking heads,
+    rep_mode 3 -- against what the reference's decode, post-process, soft-NMS and PnP returned for them."""
+    for name in ("decode_rep1_5obj", "decode_track_rep1_2obj", "decode_rep3_3obj"):
+        _check_golden(name)
 
 
 def test_pnp_matches_cv2():
@@ -112,10 +107,9 @@ def test_nms_and_topk_semantics():
     assert list(ind[0][:3]) == [14, 15, 28] and sc[0][3] == 0.0 and ind[0][3] == 0   # ties -> lowest index first
 
 
-def test_moments_matches_reference_gpfit(reference):
-    from lib.utils.gpfit import moments as ref_moments, fitgaussian
-    rng = np.random.default_rng(3)
-    for _ in range(30):
-        w = rng.random((11, 11)) * np.exp(-((np.arange(11)[:, None] - 5.3) ** 2 + (np.arange(11)[None] - 4.6) ** 2) / 6)
-        assert np.allclose(decode_ref.moments(w), ref_moments(w), rtol=0, atol=0)
-        assert np.allclose(decode_ref.moments(w), fitgaussian(w), rtol=0, atol=1e-12)
+def test_moments_matches_reference_gpfit():
+    from oracle.make_golden import gpfit_windows
+    g = golden("gpfit_moments")
+    for w, m, fit in zip(gpfit_windows(), g["moments"], g["fitgaussian"]):
+        assert np.allclose(decode_ref.moments(w), m, rtol=0, atol=0)
+        assert np.allclose(decode_ref.moments(w), fit, rtol=0, atol=1e-12)

@@ -1,6 +1,6 @@
 """Pins oracle/net_ref.py (the CPU fp32 restatement of the network) against
-(a) the golden head tensors the unmodified reference produced
-(tests/golden/net_*.npz) and (b) the live reference when it is present."""
+the golden head tensors the unmodified reference produced (tests/golden/net_*.npz),
+at the benchmarked 512 x 512 shape too."""
 import numpy as np
 import pytest
 import torch
@@ -8,7 +8,7 @@ import torch
 import centerpose_b200 as cpb
 from centerpose_b200 import synth
 from oracle import net_ref
-from tests.util import golden, net_case_inputs
+from tests.util import golden, golden_threads, net_case_inputs
 
 CASES = ["net_dla34_b2_96x128", "net_dlav1_b1_64x64", "net_dla34track_b1_64x96"]
 
@@ -20,13 +20,13 @@ def _run_oracle(g):
     sd = synth.seeded_state_dict(m, seed=int(g["wseed"]), offset_std=float(g["offset_std"]))
     x, extra = net_case_inputs(g)
     kw = {k: torch.from_numpy(v) for k, v in extra.items()}
-    return net_ref.forward(torch.from_numpy(x), sd, opt.heads, arch, **kw), opt, sd, x, extra
+    with golden_threads():
+        return net_ref.forward(torch.from_numpy(x), sd, opt.heads, arch, **kw), opt
 
 
-@pytest.mark.parametrize("name", CASES)
-def test_oracle_matches_reference_golden(name):
+def _check_golden(name):
     g = golden(name)
-    out, opt, _, _, _ = _run_oracle(g)
+    out, opt = _run_oracle(g)
     assert list(out) == list(opt.heads)
     for h in opt.heads:
         want = g["head_" + h]
@@ -35,17 +35,14 @@ def test_oracle_matches_reference_golden(name):
         assert np.abs(got - want).max() <= 2e-5 * max(1.0, np.abs(want).max()), h
 
 
-def test_oracle_matches_live_reference(reference):
-    from lib.models.model import create_model as ref_create
-    g = golden(CASES[0])
-    out, opt, sd, x, extra = _run_oracle(g)
-    ropt = reference.make_opt("dla_34")
-    ref = ref_create(ropt.arch, ropt.heads, ropt.head_conv, ropt).eval()
-    ref.load_state_dict(sd, strict=True)
-    with torch.no_grad():
-        want = ref(torch.from_numpy(x))[-1]
-    for h in want:
-        assert (want[h] - out[h]).abs().max().item() <= 2e-5 * max(1.0, want[h].abs().max().item())
+@pytest.mark.parametrize("name", CASES)
+def test_oracle_matches_reference_golden(name):
+    _check_golden(name)
+
+
+def test_oracle_matches_live_reference():
+    """At the benchmarked 512 x 512 shape: the heads the reference computed on the same seeded weights and input."""
+    _check_golden("net_dla34_b1_512")
 
 
 def test_dcn_restatement_matches_reference_cpp():

@@ -153,6 +153,20 @@ import os
 
 
 @contextlib.contextmanager
+def golden_threads():
+    """The CPU thread count the reference ran with when it wrote the fixtures (oracle/make_golden.py GOLDEN_THREADS), for
+    oracle computations that are compared with them."""
+    import torch
+    from oracle.make_golden import GOLDEN_THREADS
+    old = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(old)
+
+
+@contextlib.contextmanager
 def no_splitk():
     """The plan picks the split-K factor of the small-map convolutions from the batch size, so a frame's heads move by
     fp32 round-off (~1e-4 of their range) with the batch it sits in -- enough to flip a threshold in the tracker or to
